@@ -15,6 +15,8 @@ two half_joins, accumulable reduce, compaction).
           Rust reference cannot be built here) on the box's host cores
 
 `--impl reference` times that CPU implementation alone on the same config.
+`--dump-outputs DIR` writes the output corrections of the last timed step (either arm) as
+DIR/<field>.npy; the seeded inputs are the same from run to run, so two builds compare output for output.
 Multi-GPU (torchrun, one rank per GPU): key-sharded arrangements, NCCL
 all-to-all per exchange point, weak scaling (SF and batch grow with N).
 """
@@ -243,6 +245,31 @@ def best_oracle(B, sf_total, per_batch, n_warm, n_steps, keep_outputs_of_first=F
     return best, table, outs
 
 
+DUMP_FIELDS = ("key", "count", "sum", "flags", "time", "diff")
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, rows):
+    """Write one step's output corrections (ROUT rows) as out_dir/<field>.npy, one float64 array per
+    field of DUMP_FIELDS, rows sorted on every field so that two builds compare array for array.
+    The 128-bit SUM is rounded to float64 once; the other fields are integers below 2**53 (group
+    keys are 45 bits) and are exact.  Beyond DUMP_MAX_BYTES, a seeded sample of the rows is written."""
+    import numpy as np
+
+    order = ("key", "count", "sum_hi", "sum_lo", "flags", "time", "diff")
+    rows = rows[np.lexsort([rows[f] for f in reversed(order)])]
+    n_max = DUMP_MAX_BYTES // (8 * len(DUMP_FIELDS))
+    if len(rows) > n_max:
+        rows = rows[np.sort(np.random.default_rng(SEED).choice(len(rows), n_max, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for f in DUMP_FIELDS:
+        if f == "sum":
+            a = np.array([float((int(h) << 64) + int(lo)) for h, lo in zip(rows["sum_hi"], rows["sum_lo"])], dtype=np.float64)
+        else:
+            a = rows[f].astype(np.float64)
+        np.save(os.path.join(out_dir, f + ".npy"), a)
+
+
 def measured_peak():
     try:
         p = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -262,7 +289,10 @@ def run_reference(args, rank):
     # same workload as our arm at --gpus N (weak scaling: SF and batch grow with N)
     n = max(1, args.gpus)
     sf = sf_per_gpu(args, n) * n
-    best, table, _ = best_oracle(B, sf, ORDERS_PER_BATCH_PER_GPU * n, args.warmup, args.steps)
+    best, table, outs = best_oracle(B, sf, ORDERS_PER_BATCH_PER_GPU * n, args.warmup, args.steps,
+                                    keep_outputs_of_first=bool(args.dump_outputs))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs[args.warmup + args.steps - 1])
     cores, value, rows, secs = best["workers"], best["value"], best["rows"], best["secs"]
     sample = (f"SF={sf:g} hydrated in {best['hyd']:.1f}s (untimed), {args.steps} batches of ~{rows // max(1, args.steps)} update rows;"
               f" best of worker counts {[t['workers'] for t in table]} on {os.cpu_count()} host cores")
@@ -641,7 +671,7 @@ def run_ours(args, rank, world, local_rank):
     # and at N=1 also as the reported CPU baseline -- a bounded sample of the same workload)
     want_oracle = not args.no_cpu_baseline
     gathered = timed_out
-    if dist is not None and want_oracle:
+    if dist is not None and (want_oracle or args.dump_outputs):
         nn = torch.tensor([len(timed_out)], dtype=torch.int64, device="cuda")
         ns = [torch.zeros_like(nn) for _ in range(world)]
         dist.all_gather(ns, nn)
@@ -687,6 +717,8 @@ def run_ours(args, rank, world, local_rank):
         }
     elif rank == 0:
         line["parity"] = None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, gathered[gathered["time"] == t_first + first_timed + n_timed - 1])
     if rank == 0:
         print(json.dumps(line), flush=True)
     if dist is not None:
@@ -704,6 +736,8 @@ def main():
     ap.add_argument("--sf-multi", type=float, default=12.5, help="scale factor per GPU at N > 1 (SF=100 at N=8, configs[4])")
     ap.add_argument("--cpu-batches", type=int, default=20)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output corrections of the last timed step to DIR/<field>.npy (float64)")
     args = ap.parse_args()
     args.warmup = max(3, args.warmup)
     rank = int(os.environ.get("RANK", "0"))

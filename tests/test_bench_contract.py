@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -37,6 +39,56 @@ def test_reference_arm_other_ranks_stay_silent():
     p = run_bench("--impl", "reference", "--gpus", "2", "--sf", "1", "--steps", "3", "--warmup", "3", env=env)
     assert p.returncode == 0, p.stderr[-2000:]
     assert p.stdout.strip() == ""
+
+
+DUMP_FIELDS = ("key", "count", "sum", "flags", "time", "diff")
+
+
+def load_dump(d):
+    import numpy as np
+
+    return {f: np.load(os.path.join(d, f + ".npy")) for f in DUMP_FIELDS}
+
+
+def consolidated(dump):
+    """The dumped rows as {(key, count, sum, flags, time): diff}, equal rows summed, zero diffs dropped."""
+    acc = {}
+    for r in zip(*(dump[f].tolist() for f in DUMP_FIELDS)):
+        acc[r[:-1]] = acc.get(r[:-1], 0) + r[-1]
+    return {k: v for k, v in acc.items() if v != 0}
+
+
+def test_reference_arm_dumps_the_last_timed_step(tmp_path):
+    """--dump-outputs writes one float64 array per output field, the same from run to run."""
+    import numpy as np
+
+    args = ("--impl", "reference", "--sf", "1", "--steps", "3", "--warmup", "3", "--dump-outputs")
+    dumps = []
+    for name in ("a", "b"):
+        p = run_bench(*args, str(tmp_path / name))
+        assert p.returncode == 0, p.stderr[-2000:]
+        dumps.append(load_dump(tmp_path / name))
+    a, b = dumps
+    assert all(a[f].dtype == np.float64 and a[f].shape == a["key"].shape for f in DUMP_FIELDS)
+    assert len(a["key"]) > 0 and set(a["diff"].tolist()) <= {-1.0, 1.0}
+    assert len(set(a["time"].tolist())) == 1  # one timestamp: the last timed step's
+    assert all(np.array_equal(a[f], b[f]) for f in DUMP_FIELDS)
+    # the step before has another timestamp
+    p = run_bench("--impl", "reference", "--sf", "1", "--steps", "2", "--warmup", "3", "--dump-outputs", str(tmp_path / "c"))
+    assert p.returncode == 0, p.stderr[-2000:]
+    assert load_dump(tmp_path / "c")["time"][0] == a["time"][0] - 1
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dump_matches_the_oracle(tmp_path):
+    """The GPU arm's dump of its last timed step holds the CPU oracle's output corrections of that step."""
+    args = ("--sf", "1", "--steps", "3", "--warmup", "3", "--no-cpu-baseline", "--dump-outputs")
+    p = run_bench(*args, str(tmp_path / "gpu"))
+    assert p.returncode == 0, p.stderr[-2000:]
+    p = run_bench("--impl", "reference", *args, str(tmp_path / "cpu"))
+    assert p.returncode == 0, p.stderr[-2000:]
+    gpu, cpu = consolidated(load_dump(tmp_path / "gpu")), consolidated(load_dump(tmp_path / "cpu"))
+    assert len(cpu) > 0 and gpu == cpu
 
 
 def test_gpu_arm_fails_loudly_without_cuda():
